@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - DrQ critic grad-steps/sec on B200 (BASELINE.json metric), one JSON line on stdout.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--precision fp32|bf16]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--precision fp32|bf16] [--dump-outputs DIR]
   torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...        (N > 1)
 
 Workload = the configuration BASELINE.json's metric is quoted on ("B=256, 2x128x128 obs" = configs[2]): `async_drq_sim` with
@@ -55,6 +55,9 @@ def parse():
     ap.add_argument("--no-rlpd", dest="rlpd", action="store_false", help="draw the whole batch from the online ring (configs[1])")
     ap.add_argument("--ref-rows", type=int, default=64, help="rows of the batch the CPU reference processes per step")
     ap.add_argument("--sustain-s", type=float, default=1.0, help="length of the additional sustained run (seconds of timed steps)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the --steps timed steps, write what the last of them returned (loss / Q / lr infos, updated parameters and "
+                         "target parameters, a fixed sample of the Adam moments) as DIR/<name>.npy; the inputs depend only on the arguments")
     a = ap.parse_args()
     if a.capacity is None:
         a.capacity = 200_000 if a.cams == 2 else 100_000
@@ -277,10 +280,29 @@ class Workload:
         sync()
         t0.record()
         for _ in range(steps):
-            self.agent.update_critics(self.next_batch())
+            out = self.agent.update_critics(self.next_batch())
         t1.record()
         sync()
+        self.last_info = out[1]
         return t0.elapsed_time(t1)
+
+    def dump_outputs(self, path, moment_sample=1 << 20):
+        """What the last timed step handed back: its info scalars and the updated agent state (trainable parameters and target
+        parameters in full; the Adam moments as a fixed, seeded sample of `moment_sample` entries to stay well under 64 MB).
+        Two runs with the same arguments draw the same batches and keys, but atomic accumulations (GroupNorm statistics, split-K
+        reductions) round in a varying order, so their float outputs agree to a tolerance, not bit for bit."""
+        torch = self.torch
+        st = self.agent._store
+        out = dict(self.last_info["critic"])                                     # critic_loss, predicted_qs, target_qs
+        out.update({k: self.last_info[k] for k in ("critic_lr", "actor_lr", "temperature_lr")})
+        out.update(params=st.params[:st.n_main], target_params=st.target[:st.n_main])
+        idx = np.sort(np.random.default_rng(0).choice(st.n, min(moment_sample, st.n), replace=False))
+        idx = torch.as_tensor(idx, device=st.m.device)
+        out.update(adam_mu_sample=st.m[idx], adam_nu_sample=st.v[idx])
+        os.makedirs(path, exist_ok=True)
+        for name, v in out.items():
+            np.save(os.path.join(path, f"{name}.npy"), v.detach().float().cpu().numpy())
+        np.save(os.path.join(path, "rng.npy"), self.agent.state.rng.astype(np.float64))   # uint32 key: exact in float64
 
     def e2e_steps(self, steps, barrier=None):
         """The public-API loop with HOST buffers: every step inserts one fresh transition from host memory (pinned staging ->
@@ -304,8 +326,9 @@ class Workload:
         self.torch.cuda.synchronize()
 
 
-def measure_single_camera(args, steps=100):
+def measure_single_camera(args):
     """Supplementary measurement on BASELINE configs[1]: single camera, whole batch from one 100k ring."""
+    steps = args.steps
     w = Workload(args, 1, False, 100_000, args.batch)
     for _ in range(11):
         w.agent.update_critics(w.next_batch())
@@ -349,6 +372,8 @@ def run_b200(args):
     w0 = time.time()
     ms = w.timed_steps(args.steps, barrier)
     launches = agent.kernel_launches - launches0
+    if args.dump_outputs and rank == 0:
+        w.dump_outputs(args.dump_outputs)
     # ---- the same loop for >= sustain-s seconds: the sustained figure, and enough nvidia-smi samples under load -----------
     n_sus = max(args.steps, int(args.sustain_s * 1e3 / max(ms / args.steps, 1e-3)) + 1)
     if world > 1:

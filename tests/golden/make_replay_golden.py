@@ -1,7 +1,7 @@
 """Generate golden fixtures for the replay ring by running the REAL reference classes.
 
-Runs only in the build container (needs /root/reference).  jax / flax / gym are not
-installed there, but the reference's replay code only *imports* them and uses
+Needs a checkout of the reference repository (rail-berkeley/serl).  jax / flax / gym need not
+be installed: the reference's replay code only *imports* them and uses
 `gym.spaces.{Box,Dict}` as shape carriers, `gym.utils.seeding.np_random` for an RNG and
 `flax.core.frozen_dict.freeze/unfreeze` as a dict wrapper - so minimal import stubs (below,
 written for this script) are enough to execute the reference's own, unmodified
@@ -11,7 +11,7 @@ The reference's index stream is unseeded; we replace its `np_random` by a script
 object so the reference consumes a known sequence (including its redraw-on-invalid loop).
 
 Output: tests/golden/replay_<case>.npz  (inputs + the reference's slot contents + sampled batches).
-Usage:  python tests/golden/make_replay_golden.py
+Usage:  python tests/golden/make_replay_golden.py <reference checkout>
 """
 from __future__ import annotations
 
@@ -21,7 +21,6 @@ import types
 
 import numpy as np
 
-REF = "/root/reference/serl_launcher"
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
@@ -220,8 +219,10 @@ def make_wrap_first_case(name="wrap_first", *, cap=10, T=1, H=3, W=2, S=2, A=2, 
 
 
 if __name__ == "__main__":
+    if len(sys.argv) != 2:
+        sys.exit("usage: python tests/golden/make_replay_golden.py <reference checkout>")
     _GYM = _install_stubs()
-    sys.path.insert(0, REF)
+    sys.path.insert(0, os.path.join(os.path.abspath(sys.argv[1]), "serl_launcher"))
     # T=1 single cam with several wrap-arounds; T=2 dual-cam; tiny cap stress
     make_case("t1_cam1", cap=37, T=1, ncam=1, H=6, W=5, S=3, A=2, n_insert=150, mean_ep=7, seed=1, n_batches=2, B=16)
     make_case("t2_cam2", cap=53, T=2, ncam=2, H=4, W=4, S=2, A=3, n_insert=230, mean_ep=9, seed=2, n_batches=2, B=16)
