@@ -74,7 +74,10 @@ typedef struct serl_batch_out {
 
 /* Replaces MemoryEfficientReplayBuffer.sample (memory_efficient_replay_buffer.py:91-164) +
  * ReplayBuffer.get_iterator's device_put (replay_buffer.py:77-90) + _unpack (utils/train_utils.py:44-66)
- * + batched_random_crop (vision/data_augmentations.py:7-36, agents/continuous/drq.py:244-253). */
+ * + batched_random_crop (vision/data_augmentations.py:7-36, agents/continuous/drq.py:244-253).
+ * One-sided output: when every obs_pix[c] (or every next_pix[c]) is NULL only the other view's frames are gathered and
+ * cropped (one CTA per row and camera instead of two); only that view's crop key / explicit offsets are needed.  The
+ * reward classifier's batch (examples/async_cable_route_drq/train_reward_classifier.py) takes positive rows' next frames and negative rows' frames. */
 int serl_replay_sample_crop(const serl_replay_view* rv, const serl_sample_request* rq,
                             const serl_batch_out* out, void* stream);
 
@@ -210,6 +213,8 @@ int serl_gemm_tf32x3(const serl_gemm_desc* d, void* stream);
 #define SERL_TGEMM_EPI_LN_TANH_HEAD 2     /* ... and head_out[m, :head_n] = C[m, :] @ head_w (256, head_n) + head_b        */
 #define SERL_TGEMM_EPI_PARTIAL 4          /* k-split partial products left in the workspace [(member * splits + s)][M][N] for serl_enc_finish */
 #define SERL_TGEMM_EPI_LN_TANH_POLICY 3   /* ... two heads (means, log-stds) -> clipped std, u = mu + std * noise, act = tanh(u), logp */
+#define SERL_TGEMM_EPI_LN_RELU_HEAD 5     /* N == 256: d = (acc + bias) [* keep_mask / keep]; C = relu(LayerNorm(d) * scale + ln_bias);
+                                             head_out[m, :head_n] = C[m, :] @ head_w + head_b; optional xhat, rstd (reward classifier) */
 typedef struct serl_tgemm_problem {
   const float* A; const float* B;
   int64_t sAz, sAm, sAk, sBz, sBk, sBn;
@@ -222,6 +227,7 @@ typedef struct serl_tgemm_problem {
   float* head_out; int64_t sHeadOutZ; int32_t ld_head;  /* HEAD: (M, head_n) with row stride ld_head; POLICY: means (M, A)   */
   const float* head_w2; const float* head_b2; float* head_out2;   /* POLICY: log-std head and its raw output (M, A)        */
   const float* noise; float* act; int32_t ld_act; float* logp; float* u_out; float* std_out;   /* POLICY (Z == 1)          */
+  const uint8_t* keep_mask; float keep;          /* LN_RELU_HEAD: optional (M, 256) dropout keep mask (16-byte aligned), keep probability */
 } serl_tgemm_problem;
 typedef struct serl_tgemm_desc {
   const serl_tgemm_problem* problems; int32_t num_problems;   /* HOST array                                                */
@@ -281,6 +287,19 @@ int serl_layernorm_tanh_bwd(const float* dt, int ld_dt, const float* t, int ld_t
                             float* dscale, float* dbias, int R, int D, void* stream);
 int serl_layernorm_param_grad(const float* dy, const float* xhat, float* dscale, float* dbias, int rows_per_group, int R, int D,
                               void* stream);   /* dscale/dbias half of serl_layernorm_tanh_bwd (when it was called with NULLs) */
+/* Reward classifier hidden layer (networks/reward_classifier.py:22-26): Dense -> Dropout(keep) -> LayerNorm(eps, fast variance) -> ReLU.
+ * Forward (fp32 build; the 16-bit builds use SERL_TGEMM_EPI_LN_RELU_HEAD): z (R, D) = Dense output incl. bias,
+ * d = keep_mask ? z / keep : 0 (keep_mask NULL: d = z), out = relu(xhat * scale + bias), optional saves xhat (R, D), rstd (R).
+ * Backward (both builds): upstream gradient dt (R, D), or dlogit[r] * head_w[d] (the Dense(1) output layer, dt NULL);
+ * ReLU derivative from the saved xhat * scale + bias > 0; dy (R, D) = gradient at the LayerNorm output (for the scale / bias
+ * gradients: SERL_SMALL_GRAD_LN); dz (R, D) = gradient at z (dropout mask and 1/keep applied).  D <= 256. */
+int serl_layernorm_relu_fwd(const float* z, int ld_z, const uint8_t* keep_mask, float keep, const float* scale, const float* bias,
+                            float* out, int ld_out, float* xhat, float* rstd, int R, int D, float eps, void* stream);
+/* Dropout backward in place over n elements: x = keep_mask ? x / keep : 0 */
+int serl_dropout_bwd(float* x, const uint8_t* keep_mask, float keep, long long n, void* stream);
+int serl_layernorm_relu_bwd(const float* dt, int ld_dt, const float* dlogit, const float* head_w, const float* xhat, const float* rstd,
+                            const float* scale, const float* bias, const uint8_t* keep_mask, float keep, float* dz, float* dy,
+                            int R, int D, void* stream);
 int serl_colsum_f32(const float* x, float* out, int groups, int rows, int D, long long ld, int accumulate, void* stream);
 int serl_copy2d_f32(const float* src, long long ld_src, float* dst, long long ld_dst, int R, int D, void* stream);
 int serl_fill_f32(float* x, float v, int n, void* stream);
@@ -304,6 +323,12 @@ int serl_bc_loss(const float* mu, const float* log_std, const float* actions, fl
                  float* dmu, float* dlogstd, float* info /*2*/, int B, int A, void* stream);
 int serl_temperature_loss(const float* logp, const float* lagrange, float target_entropy, float grad_scale,
                           float* dlagrange, float* info /*1*/, int B, void* stream);
+/* Reward classifier loss (examples/async_cable_route_drq/train_reward_classifier.py:122-137): optax.sigmoid_binary_cross_entropy(x, y).mean()
+ * = mean(relu(x) - x*y + log1p(exp(-|x|))) over the train logits x (B), labels y (B);
+ * dlogit = grad_scale * (sigmoid(x) - y) / B; info[0] = loss, info[1] = mean((sigmoid(x_eval) >= 0.5) == y) over the eval
+ * logits (train=False pass, pre-update parameters), both * grad_scale.  One CTA, fixed-order reduction. */
+int serl_bce_logits_loss(const float* logits, const float* eval_logits, const float* labels, int B, float grad_scale,
+                         float* dlogit, float* info /*2*/, void* stream);
 
 /* Stride-1 3x3 convolution + GroupNorm(4 groups) [+ residual] [+ ReLU] in one kernel (vision/resnet_v1.py:129-156: the
    ResNetBlock body after / including each 3x3 conv).  An image's accumulators stay in tensor memory until its statistics are

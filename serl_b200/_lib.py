@@ -10,7 +10,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "lib", "libserl_b200.so")
 MAX_CAMS = 4
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 (KEY_CROP_OBS, KEY_CROP_NEXT, KEY_CRITIC_NEXT, KEY_CRITIC_SUBSAMPLE, KEY_ACTOR_DROPOUT, KEY_ACTOR_SAMPLE,
  KEY_TEMP_NEXT) = range(7)
@@ -57,7 +57,8 @@ class TgemmProblem(C.Structure):
                 ("C", vp), ("sCz", i64), ("ldc", i32), ("bias", vp), ("sBiasZ", i64), ("ln_scale", vp), ("ln_bias", vp), ("sLnZ", i64),
                 ("xhat", vp), ("rstd", vp), ("sXhatZ", i64), ("sRstdZ", i64), ("head_w", vp), ("head_b", vp), ("sHeadWz", i64),
                 ("sHeadBz", i64), ("head_out", vp), ("sHeadOutZ", i64), ("ld_head", i32), ("head_w2", vp), ("head_b2", vp),
-                ("head_out2", vp), ("noise", vp), ("act", vp), ("ld_act", i32), ("logp", vp), ("u_out", vp), ("std_out", vp)]
+                ("head_out2", vp), ("noise", vp), ("act", vp), ("ld_act", i32), ("logp", vp), ("u_out", vp), ("std_out", vp),
+                ("keep_mask", vp), ("keep", f32)]
 
 
 class TgemmDesc(C.Structure):
@@ -91,7 +92,7 @@ class SmallGradJob(C.Structure):
 
 
 SMALL_GRAD_COLSUM, SMALL_GRAD_LN, SMALL_GRAD_HEAD = range(3)
-TGEMM_STORE, TGEMM_LN_TANH, TGEMM_LN_TANH_HEAD, TGEMM_LN_TANH_POLICY, TGEMM_PARTIAL = range(5)
+TGEMM_STORE, TGEMM_LN_TANH, TGEMM_LN_TANH_HEAD, TGEMM_LN_TANH_POLICY, TGEMM_PARTIAL, TGEMM_LN_RELU_HEAD = range(6)
 TGEMM_MAX_PROBLEMS = 6
 
 
@@ -170,6 +171,8 @@ _PROTOS = {
     "serl_layernorm_tanh_fwd": [vp, C.c_int, vp, vp, C.c_int, C.c_int, vp, C.c_int, vp, vp, C.c_int, C.c_int, f32, vp],
     "serl_layernorm_tanh_bwd": [vp, C.c_int, vp, C.c_int, vp, vp, vp, C.c_int, C.c_int, vp, vp, vp, vp, C.c_int, C.c_int, vp],
     "serl_layernorm_param_grad": [vp, vp, vp, vp, C.c_int, C.c_int, C.c_int, vp],
+    "serl_layernorm_relu_fwd": [vp, C.c_int, vp, f32, vp, vp, vp, C.c_int, vp, vp, C.c_int, C.c_int, f32, vp],
+    "serl_layernorm_relu_bwd": [vp, C.c_int, vp, vp, vp, vp, vp, vp, vp, f32, vp, vp, C.c_int, C.c_int, vp],
     "serl_colsum_f32": [vp, vp, C.c_int, C.c_int, C.c_int, C.c_longlong, C.c_int, vp],
     "serl_copy2d_f32": [vp, C.c_longlong, vp, C.c_longlong, C.c_int, C.c_int, vp],
     "serl_fill_f32": [vp, f32, C.c_int, vp],
@@ -181,6 +184,8 @@ _PROTOS = {
     "serl_tanh_bwd": [vp, vp, vp, C.c_int, vp],
     "serl_bc_loss": [vp, vp, vp, f32, f32, f32, vp, vp, vp, C.c_int, C.c_int, vp],
     "serl_temperature_loss": [vp, vp, f32, f32, vp, vp, C.c_int, vp],
+    "serl_dropout_bwd": [vp, vp, f32, C.c_longlong, vp],
+    "serl_bce_logits_loss": [vp, vp, vp, C.c_int, f32, vp, vp, vp],
     "serl_adam_polyak": [C.POINTER(AdamDesc), vp],
 }
 EXPORTS = sorted(list(_PROTOS) + ["serl_last_error", "serl_version", "serl_device_sm_count", "serl_launch_count", "serl_stem_v2_active", "serl_balanced_grid"])

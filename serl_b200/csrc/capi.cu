@@ -56,7 +56,7 @@ int balanced_grid(int items, int sms) {
 }  // namespace serl
 
 extern "C" int serl_balanced_grid(int items, int sms) { return serl::balanced_grid(items, sms); }
-extern "C" int serl_version(void) { return 3; }
+extern "C" int serl_version(void) { return 4; }
 extern "C" unsigned long long serl_launch_count(void) { return serl::launch_count(); }
 extern "C" int serl_set_pdl(int enabled) { serl::g_pdl = enabled ? 1 : 0; return SERL_OK; }
 extern "C" int serl_device_sm_count(int device) {

@@ -171,6 +171,91 @@ __global__ void __launch_bounds__(256) ln_param_grad_kernel(const float* __restr
   }
 }
 
+// ---- reward classifier hidden layer: Dense -> Dropout -> LayerNorm -> ReLU (networks/reward_classifier.py:22-26) ----------
+// Forward, warp per row: d = keep_mask ? z / keep : 0, LayerNorm statistics of d (fast variance), out = relu(xhat*scale + bias).
+__global__ void ln_relu_fwd_kernel(const float* __restrict__ z, int ld_z, const uint8_t* __restrict__ keep_mask, float keep,
+                                   const float* __restrict__ scale, const float* __restrict__ bias, float* __restrict__ out, int ld_out,
+                                   float* __restrict__ xhat, float* __restrict__ rstd_out, int R, int D, float eps) {
+  pdl_prologue();
+  const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  const int lane = threadIdx.x & 31;
+  if (row >= R) return;
+  float v[8];
+  float s = 0.f, ss = 0.f;
+#pragma unroll
+  for (int j = 0; j < 8; ++j) {
+    const int d = lane + 32 * j;
+    v[j] = 0.f;
+    if (d < D) {
+      float x = z[(size_t)row * ld_z + d];
+      if (keep_mask) x = keep_mask[(size_t)row * D + d] ? x / keep : 0.f;
+      v[j] = x; s += x; ss += x * x;
+    }
+  }
+  s = warp_sum(s); ss = warp_sum(ss);
+  const float mean = s / (float)D;
+  const float var = fmaxf(ss / (float)D - mean * mean, 0.f);
+  const float rstd = rsqrtf(var + eps);
+#pragma unroll
+  for (int j = 0; j < 8; ++j) {
+    const int d = lane + 32 * j;
+    if (d < D) {
+      const float xh = (v[j] - mean) * rstd;
+      out[(size_t)row * ld_out + d] = fmaxf(fmaf(xh, scale[d], bias[d]), 0.f);
+      if (xhat) xhat[(size_t)row * D + d] = xh;
+    }
+  }
+  if (rstd_out && lane == 0) rstd_out[row] = rstd;
+}
+
+// Backward, warp per row (serves the fp32 chain and the LN_RELU_HEAD epilogue of tgemm.cu, which saves the same xhat / rstd):
+// dt = upstream or dlogit * w;  dy = dt * [xhat*scale + bias > 0];  dd = rstd * (dy*scale - mean(dy*scale) - xhat * mean(dy*scale*xhat));
+// dz = keep_mask ? dd / keep : 0.
+__global__ void __launch_bounds__(256) ln_relu_bwd_kernel(const float* __restrict__ dt, int ld_dt, const float* __restrict__ dlogit,
+                                                          const float* __restrict__ head_w, const float* __restrict__ xhat,
+                                                          const float* __restrict__ rstd, const float* __restrict__ scale,
+                                                          const float* __restrict__ bias, const uint8_t* __restrict__ keep_mask, float keep,
+                                                          float* __restrict__ dz, float* __restrict__ dy_out, int R, int D) {
+  pdl_prologue();
+  const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  const int lane = threadIdx.x & 31;
+  if (row >= R) return;
+  const float dl = dt ? 0.f : dlogit[row];
+  float dy[8], xh[8];
+  float m1 = 0.f, m2 = 0.f;
+#pragma unroll
+  for (int j = 0; j < 8; ++j) {
+    const int d = lane + 32 * j;
+    dy[j] = 0.f; xh[j] = 0.f;
+    if (d < D) {
+      xh[j] = xhat[(size_t)row * D + d];
+      const float g = dt ? dt[(size_t)row * ld_dt + d] : dl * head_w[d];
+      dy[j] = fmaf(xh[j], scale[d], bias[d]) > 0.f ? g : 0.f;
+      const float dxh = dy[j] * scale[d];
+      m1 += dxh; m2 += dxh * xh[j];
+      if (dy_out) dy_out[(size_t)row * D + d] = dy[j];
+    }
+  }
+  m1 = warp_sum(m1) / (float)D; m2 = warp_sum(m2) / (float)D;
+  const float rs = rstd[row];
+#pragma unroll
+  for (int j = 0; j < 8; ++j) {
+    const int d = lane + 32 * j;
+    if (d < D) {
+      float g = rs * (dy[j] * scale[d] - m1 - xh[j] * m2);
+      if (keep_mask) g = keep_mask[(size_t)row * D + d] ? g / keep : 0.f;
+      dz[(size_t)row * D + d] = g;
+    }
+  }
+}
+
+// ---- Dropout backward in place: x = mask ? x / keep : 0 (the SLE output's gradient of a train=True pass before the kernel gradient) --
+__global__ void dropout_bwd_kernel(float* __restrict__ x, const uint8_t* __restrict__ mask, float keep, long long n) {
+  pdl_prologue();
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
+    x[i] = mask[i] ? x[i] / keep : 0.f;
+}
+
 // ---- strided 2-D copy (concat helper) -------------------------------------------------------------
 __global__ void copy2d_kernel(const float* __restrict__ src, long long ld_src, float* __restrict__ dst, long long ld_dst, int R, int D) {
   pdl_prologue();
@@ -252,4 +337,30 @@ extern "C" int serl_copy2d_f32(const float* src, long long ld_src, float* dst, l
   int blocks = (int)((total + 255) / 256); if (blocks > 1184) blocks = 1184; if (blocks < 1) blocks = 1;
   launch_k(copy2d_kernel, blocks, 256, 0, ST(stream), src, ld_src, dst, ld_dst, R, D);
   return check_launch("copy2d_kernel");
+}
+
+extern "C" int serl_layernorm_relu_fwd(const float* z, int ld_z, const uint8_t* keep_mask, float keep, const float* scale, const float* bias,
+                                       float* out, int ld_out, float* xhat, float* rstd, int R, int D, float eps, void* stream) {
+  if (!z || !scale || !bias || !out || R < 1 || D < 1 || D > 256 || (keep_mask && !(keep > 0.f))) {
+    set_last_error("serl_layernorm_relu_fwd: invalid arguments (D <= 256, keep > 0 with a mask)"); return SERL_ERR_INVALID;
+  }
+  launch_k(ln_relu_fwd_kernel, ceil_div(R, 8), 256, 0, ST(stream), z, ld_z, keep_mask, keep, scale, bias, out, ld_out, xhat, rstd, R, D, eps);
+  return check_launch("ln_relu_fwd_kernel");
+}
+
+extern "C" int serl_layernorm_relu_bwd(const float* dt, int ld_dt, const float* dlogit, const float* head_w, const float* xhat, const float* rstd,
+                                       const float* scale, const float* bias, const uint8_t* keep_mask, float keep, float* dz, float* dy,
+                                       int R, int D, void* stream) {
+  if ((!dt && (!dlogit || !head_w)) || !xhat || !rstd || !scale || !bias || !dz || R < 1 || D < 1 || D > 256 || (keep_mask && !(keep > 0.f))) {
+    set_last_error("serl_layernorm_relu_bwd: invalid arguments (dt, or dlogit + head_w; D <= 256)"); return SERL_ERR_INVALID;
+  }
+  launch_k(ln_relu_bwd_kernel, ceil_div(R, 8), 256, 0, ST(stream), dt, ld_dt, dlogit, head_w, xhat, rstd, scale, bias, keep_mask, keep, dz, dy, R, D);
+  return check_launch("ln_relu_bwd_kernel");
+}
+
+extern "C" int serl_dropout_bwd(float* x, const uint8_t* keep_mask, float keep, long long n, void* stream) {
+  if (!x || !keep_mask || n < 1 || !(keep > 0.f)) { set_last_error("serl_dropout_bwd: invalid arguments"); return SERL_ERR_INVALID; }
+  long long blocks = (n + 255) / 256; if (blocks > 2368) blocks = 2368;
+  launch_k(dropout_bwd_kernel, (int)blocks, 256, 0, ST(stream), x, keep_mask, keep, n);
+  return check_launch("dropout_bwd_kernel");
 }

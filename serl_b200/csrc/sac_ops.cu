@@ -299,6 +299,31 @@ __global__ void __launch_bounds__(1024) bc_loss_kernel(const float* __restrict__
   if (threadIdx.x == 0) { info[0] = sl * inv; info[1] = sm * inv; }
 }
 
+// ---------------------------------------------------------------------------------------------
+// Reward classifier (examples/async_cable_route_drq/train_reward_classifier.py:122-137): optax.sigmoid_binary_cross_entropy(x, y).mean()
+// restated in the stable form relu(x) - x*y + log1p(exp(-|x|)); gradient (sigmoid(x) - y) / B.  Accuracy is the reference's
+// predicate (nn.sigmoid(logit) >= 0.5) == label evaluated literally in fp32 on the eval logit: 1 / (1 + expf(-x)) >= 0.5f, which
+// holds for every x >= 0 AND for negative x with |x| < ~6e-8 (expf(-x) rounds to 1 there), like the reference's fp32 sigmoid.
+// info[0] = loss, info[1] = accuracy (both * grad_scale, see critic_loss_kernel); one CTA, fixed-order reduction (no atomics).
+// ---------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(1024) bce_logits_loss_kernel(const float* __restrict__ x, const float* __restrict__ xe,
+                                                               const float* __restrict__ y, int B, float grad_scale,
+                                                               float* __restrict__ dlogit, float* __restrict__ info) {
+  pdl_prologue();
+  __shared__ float red[64];
+  float sl = 0.f, sa = 0.f;
+  const float inv = grad_scale / (float)B;
+  for (int b = threadIdx.x; b < B; b += blockDim.x) {
+    const float v = x[b], lab = y[b];
+    sl += fmaxf(v, 0.f) - v * lab + log1pf(expf(-fabsf(v)));
+    dlogit[b] = (1.f / (1.f + expf(-v)) - lab) * inv;
+    const bool pred = 1.f / (1.f + expf(-xe[b])) >= 0.5f;
+    sa += ((pred ? 1.f : 0.f) == lab) ? 1.f : 0.f;
+  }
+  block_sum2(sl, sa, red);
+  if (threadIdx.x == 0) { info[0] = sl * inv; info[1] = sa * inv; }
+}
+
 __global__ void adam_tick_kernel(const AdamArgs a) {
   pdl_prologue();
   const int gid = threadIdx.x;
@@ -421,4 +446,11 @@ extern "C" int serl_adam_polyak(const serl_adam_desc* d, void* stream) {
   if (int e = check_launch("adam_polyak_kernel")) return e;
   launch_k(adam_tick_kernel, 1, 32, 0, ST(stream), a);
   return check_launch("adam_tick_kernel");
+}
+
+extern "C" int serl_bce_logits_loss(const float* logits, const float* eval_logits, const float* labels, int B, float grad_scale,
+                                    float* dlogit, float* info, void* stream) {
+  if (!logits || !eval_logits || !labels || !dlogit || !info || B < 1) { set_last_error("serl_bce_logits_loss: invalid arguments"); return SERL_ERR_INVALID; }
+  launch_k(bce_logits_loss_kernel, 1, 1024, 0, ST(stream), logits, eval_logits, labels, B, grad_scale, dlogit, info);
+  return check_launch("bce_logits_loss_kernel");
 }

@@ -44,6 +44,7 @@ struct SamplerArgs {
   uint8_t* dones; int32_t* idx_out; int32_t* off_obs_out; int32_t* off_next_out;   // off_*: (B_total*T, 2)
   int32_t* status;               // device int, OR-ed with 1 when a draw fails
   int batch;                     // rows produced by this launch
+  int one_side;                  // 0: obs and next frames; 1: obs frames only; 2: next frames only (the other side's pointers are NULL)
 };
 
 __device__ inline int draw_index(const SamplerArgs& a, uint32_t lane) {
@@ -102,14 +103,15 @@ __global__ void __launch_bounds__(kSamplerThreads) sample_gather_crop_kernel(con
   const int band = blockIdx.x;
   int yz = blockIdx.y;
   const int t = yz % T; yz /= T;
-  const int which = yz & 1; yz >>= 1;
+  const int which = a.one_side ? a.one_side - 1 : (yz & 1);
+  if (!a.one_side) yz >>= 1;
   const int cam = yz;
   const int i = blockIdx.z;
   const int out_row = a.out_row_offset + i;
   const int g = out_row * T + t;                         // frame index inside the batch
   const int y0 = band * kBandRows;
   const int rows = min(kBandRows, H - y0);
-  const bool leader = (cam == 0 && which == 0 && t == 0 && band == 0);
+  const bool leader = (cam == 0 && (which == 0 || a.one_side) && t == 0 && band == 0);
 
   if (threadIdx.x == 0) {
     int idx = a.explicit_idx ? a.explicit_idx[i] : draw_index(a, a.lane_offset + (uint32_t)i);
@@ -243,7 +245,7 @@ __device__ inline void crop_offset_warp(const uint32_t* key, const int32_t* expl
   *cx = (int)(((hb1 % sp) * mult + (lb1 % sp)) % sp);
 }
 
-// grid: x = cam*2 + which, y = row i.
+// grid: x = cam*2 + which (one-sided: x = cam), y = row i.
 __global__ void __launch_bounds__(kFrameThreads) sample_frames_kernel(const SamplerArgs a) {
   pdl_prologue();
   extern __shared__ __align__(128) uint8_t smem[];
@@ -253,11 +255,11 @@ __global__ void __launch_bounds__(kFrameThreads) sample_frames_kernel(const Samp
   const serl_replay_view& rv = a.rv;
   const int T = rv.num_stack, H = rv.height, W = rv.width, C = rv.channels;
   const int row_bytes = W * C;
-  const int which = blockIdx.x & 1, cam = blockIdx.x >> 1;
+  const int which = a.one_side ? a.one_side - 1 : (blockIdx.x & 1), cam = a.one_side ? blockIdx.x : (blockIdx.x >> 1);
   const int i = blockIdx.y;
   const int out_row = a.out_row_offset + i;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const bool leader = (cam == 0 && which == 0);
+  const bool leader = (cam == 0 && (which == 0 || a.one_side));
   const int band_bytes = kBandRows * row_bytes + 32;
 
   if (threadIdx.x == 0) {
@@ -641,9 +643,24 @@ extern "C" int serl_replay_sample_crop(const serl_replay_view* rv, const serl_sa
     set_last_error("serl_replay_sample_crop: buffer holds %d slots, need > num_stack", rv->size);
     return SERL_ERR_INVALID;
   }
-  if (rv->num_cams > 0 && (!rq->key_obs || !rq->key_next) && (!rq->explicit_off_obs || !rq->explicit_off_next)) {
-    set_last_error("serl_replay_sample_crop: need crop keys or explicit offsets");
-    return SERL_ERR_INVALID;
+  // one-sided output: every obs_pix (or every next_pix) pointer NULL -> only the other view is gathered and cropped, one CTA per
+  // (row, camera) instead of two (the reward classifier's batch uses the positive rows' next frames and the negative rows' frames)
+  int one_side = 0;
+  if (rv->num_cams > 0) {
+    bool any_obs = false, any_next = false;
+    for (int c = 0; c < rv->num_cams; ++c) { any_obs |= out->obs_pix[c] != nullptr; any_next |= out->next_pix[c] != nullptr; }
+    if (!any_obs && !any_next) { set_last_error("serl_replay_sample_crop: no frame output"); return SERL_ERR_INVALID; }
+    one_side = any_obs && any_next ? 0 : (any_obs ? 1 : 2);
+    for (int c = 0; c < rv->num_cams; ++c)
+      if ((one_side != 2 && !out->obs_pix[c]) || (one_side != 1 && !out->next_pix[c])) {
+        set_last_error("serl_replay_sample_crop: camera %d: frame output missing", c); return SERL_ERR_INVALID;
+      }
+    const bool obs_ok = rq->key_obs || rq->explicit_off_obs, next_ok = rq->key_next || rq->explicit_off_next;
+    const bool two_ok = (rq->key_obs && rq->key_next) || (rq->explicit_off_obs && rq->explicit_off_next);
+    if (one_side == 0 ? !two_ok : (one_side == 1 ? !obs_ok : !next_ok)) {
+      set_last_error("serl_replay_sample_crop: need crop keys or explicit offsets");
+      return SERL_ERR_INVALID;
+    }
   }
   SamplerArgs a{};
   a.rv = *rv;
@@ -655,10 +672,12 @@ extern "C" int serl_replay_sample_crop(const serl_replay_view* rv, const serl_sa
   a.obs_state = out->obs_state; a.next_state = out->next_state; a.actions = out->actions;
   a.rewards = out->rewards; a.masks = out->masks; a.dones = out->dones; a.idx_out = out->idx;
   a.off_obs_out = out->off_obs; a.off_next_out = out->off_next; a.status = out->status; a.batch = rq->batch;
+  a.one_side = one_side;
+  const int sides = one_side ? 1 : 2;
 
   const int row_bytes = rv->width * rv->channels;
   const bool fast = rv->num_cams > 0 && (row_bytes % 16 == 0) && ((reinterpret_cast<uintptr_t>(rv->frames[0]) & 15) == 0);
-  dim3 grid(ceil_div(rv->height, kBandRows), rv->num_cams * 2 * rv->num_stack, rq->batch);
+  dim3 grid(ceil_div(rv->height, kBandRows), rv->num_cams * sides * rv->num_stack, rq->batch);
   if (rv->num_cams == 0) grid = dim3(1, 1, rq->batch);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (fast && rv->num_stack <= 8 && ceil_div(rv->height, kBandRows) <= kMaxBands &&
@@ -671,7 +690,7 @@ extern "C" int serl_replay_sample_crop(const serl_replay_view* rv, const serl_sa
     }
     static int persistent = -1;
     if (persistent < 0) { const char* e = getenv("SERL_SAMPLER_PERSISTENT"); persistent = (e && atoi(e) != 0) ? 1 : 0; }
-    if (persistent && rv->num_stack == 1 && 2 * smem <= 112 * 1024) {
+    if (persistent && !one_side && rv->num_stack == 1 && 2 * smem <= 112 * 1024) {
       static int sms = 0;
       if (!sms) { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev); if (sms <= 0) sms = 148; }
       const int n_items = rq->batch * rv->num_cams * 2;
@@ -685,7 +704,7 @@ extern "C" int serl_replay_sample_crop(const serl_replay_view* rv, const serl_sa
       launch_k(sample_frames_persistent_kernel, grid, kFrameThreads, 2 * smem, st, a, n_items);
       return check_launch("sample_frames_persistent_kernel");
     }
-    dim3 fgrid(rv->num_cams * 2, rq->batch);
+    dim3 fgrid(rv->num_cams * sides, rq->batch);
     launch_k(sample_frames_kernel, fgrid, kFrameThreads, smem, st, a);
     return check_launch("sample_frames_kernel");
   } else if (fast) {

@@ -11,7 +11,9 @@
 //   * fused epilogues: bias; bias + LayerNorm(eps 1e-6, fast variance) + tanh with the statistics the backward pass needs
 //     (an output row is one TMEM lane, so the row reductions are thread-local); + the value head (Q = h . w + b,
 //     networks/actor_critic_nets.py:64-72) or the policy's mean / log-std heads with the tanh-Gaussian sample and its
-//     log-probability (actor_critic_nets.py:187-227, 230-272) in the same pass.
+//     log-probability (actor_critic_nets.py:187-227, 230-272) in the same pass;
+//   * the reward classifier's hidden layer (networks/reward_classifier.py:22-28): bias + Dropout keep mask + LayerNorm + ReLU and
+//     the Dense(1) logit head in one epilogue (LN_RELU_HEAD; train pass with the mask and eval pass without it = two problems).
 // Accuracy: TF32 operands (10-bit mantissa, round to nearest), fp32 accumulation - what XLA's default matmul precision gives
 // the reference on an NVIDIA GPU; the 16-bit builds are held to 1e-2 (north_star), the fp32 build keeps the SGEMM heads.
 // Up to TG_MAXG problem groups (e.g. the three encoder passes x two cameras of a critic step) share one launch.
@@ -39,6 +41,7 @@ struct TgGroup {
   const float* head_w; const float* head_b; float* head_out;
   const float* head_w2; const float* head_b2; float* head_out2;
   const float* noise; float* act; float* logp; float* u_out; float* std_out;
+  const uint8_t* keep_mask; float keep;
   long long sCz, sBiasZ, sLnZ, sXhatZ, sRstdZ, sHeadWz, sHeadBz, sHeadOutZ;
   int ldc, ld_head, ld_act, z0, Z, a_bcast, b_bcast;
 };
@@ -107,6 +110,8 @@ __device__ inline void tg_ld32(uint32_t taddr, float (&v)[32]) {
 __device__ inline float tg_tanh(float x) { return 1.f - __fdividef(2.f, __expf(2.f * x) + 1.f); }
 __device__ inline float tg_softplus(float x) { return fmaxf(x, 0.f) + log1pf(expf(-fabsf(x))); }
 
+// kRelu: the LN_RELU_HEAD instantiation; every other epilogue runs the kRelu = false instantiation, whose code is the tanh epilogues' alone
+template <bool kRelu>
 __global__ void __launch_bounds__(TG_THREADS, 1) tgemm_tf32_kernel(const __grid_constant__ TgMaps maps, const __grid_constant__ TgArgs a) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
@@ -209,7 +214,8 @@ __global__ void __launch_bounds__(TG_THREADS, 1) tgemm_tf32_kernel(const __grid_
     const int hh = (warp - 2) >> 2;                                      // column half
     const int row = q * 32 + lane, m = m0 + row;
     const int c_lo = hh * (TG_BN / 2), c_hi = c_lo + TG_BN / 2;
-    const bool ln = a.epi >= SERL_TGEMM_EPI_LN_TANH && a.epi <= SERL_TGEMM_EPI_LN_TANH_POLICY;
+    constexpr bool relu = kRelu;
+    const bool ln = (a.epi >= SERL_TGEMM_EPI_LN_TANH && a.epi <= SERL_TGEMM_EPI_LN_TANH_POLICY) || relu;
     // stage the epilogue vectors while the main loop runs
     if (!a.to_ws) {
       const float* bias = g.bias ? g.bias + z * g.sBiasZ : nullptr;
@@ -294,14 +300,32 @@ __global__ void __launch_bounds__(TG_THREADS, 1) tgemm_tf32_kernel(const __grid_
         }
       }
     } else {
-      // ---- bias + LayerNorm + tanh (N == 256: a row = this thread's 128 columns + its partner's) ----
+      // ---- bias [+ dropout] + LayerNorm + tanh | ReLU (N == 256: a row = this thread's 128 columns + its partner's) ----
+      // LN_RELU_HEAD with a keep mask: d = mask ? (acc + bias) / keep : 0 (flax Dropout), applied before the statistics
+      const uint8_t* mrow = (relu && g.keep_mask && m < a.M) ? g.keep_mask + (size_t)m * TG_BN : nullptr;
+      auto drop = [&](float (&v)[32], int c) {
+        if (relu && mrow) {
+          const uint4 b0 = *reinterpret_cast<const uint4*>(mrow + c), b1 = *reinterpret_cast<const uint4*>(mrow + c + 16);
+          const uint32_t w[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
+#pragma unroll
+          for (int i = 0; i < 32; ++i) v[i] = ((w[i >> 2] >> (8 * (i & 3))) & 0xffu) ? v[i] / g.keep : 0.f;
+        }
+      };
       float s = 0.f, ss = 0.f;
 #pragma unroll 1
       for (int c = c_lo; c < c_hi; c += 32) {
         float v[32];
         tg_ld32(tbase + (uint32_t)c, v);
+        if constexpr (relu) {
 #pragma unroll
-        for (int i = 0; i < 32; ++i) { const float x = v[i] + sBias[c + i]; s += x; ss += x * x; }
+          for (int i = 0; i < 32; ++i) v[i] += sBias[c + i];
+          drop(v, c);
+#pragma unroll
+          for (int i = 0; i < 32; ++i) { const float x = v[i]; s += x; ss += x * x; }
+        } else {
+#pragma unroll
+          for (int i = 0; i < 32; ++i) { const float x = v[i] + sBias[c + i]; s += x; ss += x * x; }
+        }
       }
       *reinterpret_cast<float2*>(sPart + (hh * TG_BM + row) * 2) = make_float2(s, ss);
       asm volatile("bar.sync 1, 256;" ::: "memory");
@@ -326,11 +350,23 @@ __global__ void __launch_bounds__(TG_THREADS, 1) tgemm_tf32_kernel(const __grid_
         float v[32];
         tg_ld32(tbase + (uint32_t)c, v);
         float h[32];
+        if constexpr (relu) {
 #pragma unroll
-        for (int i = 0; i < 32; ++i) {
-          const float xh = (v[i] + sBias[c + i] - mean) * rstd;
-          v[i] = xh;
-          h[i] = tg_tanh(fmaf(xh, sLs[c + i], sLb[c + i]));
+          for (int i = 0; i < 32; ++i) v[i] += sBias[c + i];
+          drop(v, c);
+#pragma unroll
+          for (int i = 0; i < 32; ++i) {
+            const float xh = (v[i] - mean) * rstd;
+            v[i] = xh;
+            h[i] = fmaxf(fmaf(xh, sLs[c + i], sLb[c + i]), 0.f);
+          }
+        } else {
+#pragma unroll
+          for (int i = 0; i < 32; ++i) {
+            const float xh = (v[i] + sBias[c + i] - mean) * rstd;
+            v[i] = xh;
+            h[i] = tg_tanh(fmaf(xh, sLs[c + i], sLb[c + i]));
+          }
         }
         if (hbase) {
           if (hvec) { stage(sTile, h); flush(sTile, hbase, g.ldc, c, false, have); }
@@ -369,7 +405,7 @@ __global__ void __launch_bounds__(TG_THREADS, 1) tgemm_tf32_kernel(const __grid_
         }
       }
       if (valid && hh == 0) {
-        if (a.epi == SERL_TGEMM_EPI_LN_TANH_HEAD) {
+        if (a.epi == SERL_TGEMM_EPI_LN_TANH_HEAD || relu) {
           float* o = g.head_out + z * g.sHeadOutZ + (size_t)m * g.ld_head;
 #pragma unroll
           for (int j = 0; j < TG_MAXHEAD; ++j) if (j < a.head_n) o[j] = hacc[j] + sHb[j];
@@ -456,14 +492,16 @@ extern "C" int serl_tgemm_tf32(const serl_tgemm_desc* d, void* stream) {
   if (!tg_get_encode()) { set_last_error("serl_tgemm_tf32: cuTensorMapEncodeTiled unavailable"); return SERL_ERR_CUDA; }
   static bool attr_done = false;
   if (!attr_done) {
-    if (cudaFuncSetAttribute(tgemm_tf32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TG_SMEM) != cudaSuccess) {
+    if (cudaFuncSetAttribute(tgemm_tf32_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TG_SMEM) != cudaSuccess ||
+        cudaFuncSetAttribute(tgemm_tf32_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TG_SMEM) != cudaSuccess) {
       set_last_error("serl_tgemm_tf32: cannot reserve %d bytes of shared memory", TG_SMEM); return SERL_ERR_CUDA;
     }
     attr_done = true;
   }
-  const bool ln = d->epilogue >= SERL_TGEMM_EPI_LN_TANH && d->epilogue <= SERL_TGEMM_EPI_LN_TANH_POLICY;
+  const bool relu = d->epilogue == SERL_TGEMM_EPI_LN_RELU_HEAD;
+  const bool ln = (d->epilogue >= SERL_TGEMM_EPI_LN_TANH && d->epilogue <= SERL_TGEMM_EPI_LN_TANH_POLICY) || relu;
   const bool partial = d->epilogue == SERL_TGEMM_EPI_PARTIAL;
-  if (d->epilogue < 0 || d->epilogue > SERL_TGEMM_EPI_PARTIAL) { set_last_error("serl_tgemm_tf32: unknown epilogue %d", d->epilogue); return SERL_ERR_INVALID; }
+  if (d->epilogue < 0 || d->epilogue > SERL_TGEMM_EPI_LN_RELU_HEAD) { set_last_error("serl_tgemm_tf32: unknown epilogue %d", d->epilogue); return SERL_ERR_INVALID; }
   if (ln && (d->N != TG_BN || d->reduce_z || d->splits > 1)) { set_last_error("serl_tgemm_tf32: LayerNorm epilogues need N == 256, no k-split, no reduce_z"); return SERL_ERR_UNSUPPORTED; }
   if (ln && d->epilogue >= SERL_TGEMM_EPI_LN_TANH_HEAD && (d->head_n < 1 || d->head_n > TG_MAXHEAD)) { set_last_error("serl_tgemm_tf32: head_n in [1, 8]"); return SERL_ERR_UNSUPPORTED; }
   TgMaps maps;
@@ -486,6 +524,10 @@ extern "C" int serl_tgemm_tf32(const serl_tgemm_desc* d, void* stream) {
     g.C = p.C; g.bias = p.bias; g.ln_scale = p.ln_scale; g.ln_bias = p.ln_bias; g.xhat = p.xhat; g.rstd = p.rstd;
     g.head_w = p.head_w; g.head_b = p.head_b; g.head_out = p.head_out; g.head_w2 = p.head_w2; g.head_b2 = p.head_b2; g.head_out2 = p.head_out2;
     g.noise = p.noise; g.act = p.act; g.logp = p.logp; g.u_out = p.u_out; g.std_out = p.std_out;
+    g.keep_mask = relu ? p.keep_mask : nullptr; g.keep = p.keep;
+    if (g.keep_mask && (!(p.keep > 0.f) || (reinterpret_cast<uintptr_t>(p.keep_mask) & 15) || p.Z != 1)) {
+      set_last_error("serl_tgemm_tf32: problem %d: keep_mask needs keep > 0, 16-byte alignment and Z == 1", i); return SERL_ERR_INVALID;
+    }
     g.sCz = p.sCz; g.sBiasZ = p.sBiasZ; g.sLnZ = p.sLnZ; g.sXhatZ = p.sXhatZ; g.sRstdZ = p.sRstdZ; g.sHeadWz = p.sHeadWz; g.sHeadBz = p.sHeadBz;
     g.sHeadOutZ = p.sHeadOutZ; g.ldc = p.ldc; g.ld_head = p.ld_head; g.ld_act = p.ld_act; g.z0 = ztotal; g.Z = p.Z;
     if (!d->reduce_z && !p.C && !ln && !partial) { set_last_error("serl_tgemm_tf32: problem %d: C required", i); return SERL_ERR_INVALID; }
@@ -526,7 +568,8 @@ extern "C" int serl_tgemm_tf32(const serl_tgemm_desc* d, void* stream) {
   a.ws = d->workspace;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   dim3 grid(ceil_div(d->M, TG_BM), ceil_div(d->N, TG_BN), ztotal * S);
-  launch_k(tgemm_tf32_kernel, grid, TG_THREADS, TG_SMEM, st, maps, a);
+  if (relu) launch_k(tgemm_tf32_kernel<true>, grid, TG_THREADS, TG_SMEM, st, maps, a);
+  else launch_k(tgemm_tf32_kernel<false>, grid, TG_THREADS, TG_SMEM, st, maps, a);
   if (int e = check_launch("tgemm_tf32_kernel")) return e;
   if (a.to_ws && !partial) {
     const serl_tgemm_problem& p = d->problems[0];

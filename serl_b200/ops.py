@@ -118,6 +118,23 @@ def ln_tanh_bwd(dt, ld_dt, t, ld_t, xhat, rstd, scale, rows_per_group, group_str
            dbias, R, D, _s())
 
 
+def ln_relu_fwd(z, ld_z, keep_mask, keep, scale, bias, out, ld_out, xhat, rstd, R, D, eps=1e-6):
+    """Dense output z -> [dropout] -> LayerNorm -> ReLU (reward classifier hidden layer); addresses, keep_mask may be None."""
+    L.call("serl_layernorm_relu_fwd", z, ld_z, keep_mask, float(keep), scale, bias, out, ld_out, xhat, rstd, R, D, float(eps), _s())
+
+
+def ln_relu_bwd(dt, ld_dt, dlogit, head_w, xhat, rstd, scale, bias, keep_mask, keep, dz, dy, R, D):
+    L.call("serl_layernorm_relu_bwd", dt, ld_dt, dlogit, head_w, xhat, rstd, scale, bias, keep_mask, float(keep), dz, dy, R, D, _s())
+
+
+def dropout_bwd(x, keep_mask, keep, n):
+    L.call("serl_dropout_bwd", x, keep_mask, float(keep), int(n), _s())
+
+
+def bce_logits_loss(logits, eval_logits, labels, B, grad_scale, dlogit, info):
+    L.call("serl_bce_logits_loss", logits, eval_logits, labels, B, float(grad_scale), dlogit, info, _s())
+
+
 def ln_param_grad(dy, xhat, dscale, dbias, rows_per_group, R, D):
     L.call("serl_layernorm_param_grad", dy, xhat, dscale, dbias, rows_per_group, R, D, _s())
 
@@ -200,7 +217,7 @@ def adam_polyak(params, target, m, v, grad, seg_end: Sequence[int], live: Sequen
 def tgemm_problem(A, B, *, sAm, sAk, sBk, sBn, Z=1, sAz=0, sBz=0, C_=None, sCz=0, ldc=0, bias=None, sBiasZ=0, ln_scale=None,
                   ln_bias=None, sLnZ=0, xhat=None, rstd=None, sXhatZ=0, sRstdZ=0, head_w=None, head_b=None, sHeadWz=0, sHeadBz=0,
                   head_out=None, sHeadOutZ=0, ld_head=1, head_w2=None, head_b2=None, head_out2=None, noise=None, act=None, ld_act=0,
-                  logp=None, u_out=None, std_out=None):
+                  logp=None, u_out=None, std_out=None, keep_mask=None, keep=1.0):
     """One problem of a serl_tgemm_tf32 launch; every operand is a device ADDRESS (int) or None, strides in floats."""
     p = L.TgemmProblem()
     p.A, p.B, p.sAz, p.sAm, p.sAk, p.sBz, p.sBk, p.sBn, p.Z = A, B, sAz, sAm, sAk, sBz, sBk, sBn, Z
@@ -209,6 +226,7 @@ def tgemm_problem(A, B, *, sAm, sAk, sBk, sBn, Z=1, sAz=0, sBz=0, C_=None, sCz=0
     p.head_w, p.head_b, p.sHeadWz, p.sHeadBz, p.head_out, p.sHeadOutZ, p.ld_head = head_w, head_b, sHeadWz, sHeadBz, head_out, sHeadOutZ, ld_head
     p.head_w2, p.head_b2, p.head_out2 = head_w2, head_b2, head_out2
     p.noise, p.act, p.ld_act, p.logp, p.u_out, p.std_out = noise, act, ld_act, logp, u_out, std_out
+    p.keep_mask, p.keep = keep_mask, float(keep)
     return p
 
 
